@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo (sm_100a kernels through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU kernels on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write each timed search path's last-step results as DIR/*.npy
 
 ONE JSON line on stdout (rank 0). The headline fields are BASELINE `configs[1]` (workload `c2`); `"configs": {"c1": …, "c3": …,
 "c4": …, "c5": …}` carries the other four, each with value / e2e / roofline / cpu_baseline / parity, so every BASELINE config has a
@@ -50,6 +51,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 SEED = 20260922
 LATENT = 32      # intrinsic dimensionality of the synthetic embedding model
 NOISE = 0.25     # isotropic noise relative to the per-coordinate signal
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this much in all; larger outputs are dumped as a fixed, seeded sample of their rows
 IMMA_PEAK_TOPS = 917.0   # tools/micro/imma_rate.cu on B200: legacy IMMA.16832 issue rate, 2*16*8*32 ops each (profiles/r2_imma_rate.md)
 UMMA_I8_PEAK_TOPS = 4559.0  # tools/micro/umma_rate.cu on B200: tcgen05.mma kind::i8 128x256x32 at 128 cycles each on all 148 SMs
 
@@ -197,6 +199,7 @@ class Ctx:
         self.lib = nat.init(self.local)
         self.VSF = jv.VectorSimilarityFunction
         self.sampler = ClockSampler(self.local)
+        self.outputs = {}  # name -> what a timed path returned in its last step (--dump-outputs)
 
     def barrier(self):
         if self.td is not None:
@@ -420,6 +423,7 @@ def bench_c2(cx, w):
     a = cx.args
     topK, rerankK = a.topk, a.topk * a.overquery
     r = search_legs(cx, w, w.vec, None, topK, rerankK, a.steps, a.warmup)
+    cx.outputs.update(c2_nodes=r["nodes"], c2_scores=r["scores"])
     total_q = a.steps * a.nq * cx.world
     peak, peak_src = measured_peaks()
     per_unit = a.dim * 4 + 8
@@ -543,6 +547,7 @@ def bench_c3(cx, w, steps):
     pqv = jv.PQVectors(codes, cb, a.dim, 256)
     w.gi.fuse_pq(pqv)
     r = search_legs(cx, w, pqv, w.vec, topK, rerankK, steps, 3)
+    cx.outputs.update(c3_nodes=r["nodes"], c3_scores=r["scores"])
     total_q = steps * a.nq * cx.world
     peak, peak_src = measured_peaks()
     adc = (r["visited"] + a.nq) * steps  # this rank
@@ -601,6 +606,7 @@ def bench_c1(cx, steps):
         nodes, _, _ = jv.topk_bruteforce(vec, VSF.EUCLIDEAN, queries, 100)
         t_bf += time.perf_counter() - t0
     launches = lib.jv_kernel_launch_count() - l0
+    cx.outputs.update(c1_nodes=res.nodes, c1_scores=res.scores, c1_bruteforce_nodes=nodes)
     peak, _ = measured_peaks()
     out = {"metric": "queries_per_sec_at_recall@100", "unit": "queries/s", "n_gpus": 1, "steps": steps, "warmup": 3, "higher_is_better": True,
            "dtype": "f32", "data": "siftsmall (tests/golden/siftsmall)",
@@ -670,6 +676,8 @@ def bench_c4(cx, steps):
     cx.barrier()
     dev_s = ev0.elapsed_time(ev1) / 1e3
     launches = lib.jv_kernel_launch_count() - l0
+    c4_nodes, c4_scores = par.keys_to_nodes_scores(keys.cpu().numpy())
+    cx.outputs.update(c4_nodes=c4_nodes, c4_scores=c4_scores)
     unresolved = sb.status()
     # e2e: host queries in (pinned), host keys out
     hq = torch.from_numpy(queries).pin_memory()
@@ -820,6 +828,19 @@ def bench_c5(cx):
 
 
 # ------------------------------------------------------------------------------------------------ driver
+def dump_outputs(d, outputs):
+    """outputs as d/<name>.npy: integer arrays (node ids) as float64, which holds them exactly, the rest as float32. Over DUMP_BYTES
+    in all, every array keeps the same fraction of its rows, a seeded sample: the same rows for every array with as many rows."""
+    os.makedirs(d, exist_ok=True)
+    arrays = {k: np.asarray(a).astype(np.float64 if np.asarray(a).dtype.kind in "iu" else np.float32) for k, a in outputs.items()}
+    frac = min(1.0, DUMP_BYTES / max(1, sum(a.nbytes for a in arrays.values())))
+    for name, a in sorted(arrays.items()):
+        if frac < 1.0:
+            a = a[np.sort(np.random.default_rng(SEED).choice(len(a), max(1, int(len(a) * frac)), replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+    log("dumped %s to %s" % (", ".join(sorted(outputs)), d))
+
+
 def guarded(name, fn):
     t0 = time.time()
     try:
@@ -855,6 +876,8 @@ def main():
                     "(ncu --profile-from-start off then lists exactly the launches of the timed region)")
     ap.add_argument("--sweep", action="store_true", help="also report overquery 1/2/5/10")
     ap.add_argument("--dist", default="latent", choices=["latent", "iid"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what each timed search path returned in its last step as "
+                    "DIR/<config>_<name>.npy (ids as float64, scores as float32; rank 0). c5's graph build is not dumped")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
 
@@ -888,6 +911,7 @@ def main():
             last = cpu_search(base, gh, w.queries[:nqs], topK, rerankK, int(VSF.DOT_PRODUCT), None, threads=nthreads)
             secs += last["seconds"]
             scored += last["scored"]
+        cx.outputs.update(c2_nodes=last["nodes"], c2_scores=last["scores"])
         qps = args.steps * nqs / secs
         out = {"metric": "queries_per_sec_at_recall@10", "unit": "queries/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
@@ -901,6 +925,8 @@ def main():
                "e2e": {"value": qps, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
                "gpu_launches": 0, "setup": "rows and graph produced on the device (untimed); the timed path is CPU only"}
         cx.sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, cx.outputs)
         print(json.dumps(out), flush=True)
         return 0
 
@@ -923,7 +949,7 @@ def main():
             if cx.rank == 0 and not args.no_cpu:
                 cb, _ = cpu_baseline_search(cx, w, args.topk, args.topk * args.overquery, None)
                 out["cpu_baseline"] = cb
-        c3 = guarded("c3", lambda: bench_c3(cx, w, max(3, min(args.steps, 10)))) if single in (None, "c3") else None
+        c3 = guarded("c3", lambda: bench_c3(cx, w, args.steps)) if single in (None, "c3") else None
         if single == "c3":
             out = c3
         elif c3 is not None:
@@ -933,13 +959,13 @@ def main():
         del w
         cx.torch.cuda.empty_cache()
     if single in (None, "c1") and cx.rank == 0:
-        c1 = guarded("c1", lambda: bench_c1(cx, max(3, min(args.steps, 10))))
+        c1 = guarded("c1", lambda: bench_c1(cx, args.steps))
         if single == "c1":
             out = c1
         else:
             out.setdefault("configs", {})["c1"] = c1
     if single in (None, "c4"):
-        c4 = guarded("c4", lambda: bench_c4(cx, max(10, args.steps)))
+        c4 = guarded("c4", lambda: bench_c4(cx, args.steps))
         if single == "c4":
             out = c4
         else:
@@ -964,6 +990,8 @@ def main():
             par.update({k: (v.get("parity", {}) or {}).get("ok") for k, v in out["configs"].items()})
             out["parity_all_ok"] = all(v is True for v in par.values())
             out["parity_by_config"] = par
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, cx.outputs)
         print(json.dumps(out), flush=True)
     if cx.td is not None:
         cx.td.destroy_process_group()

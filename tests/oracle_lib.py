@@ -149,52 +149,39 @@ def load():
     return L
 
 
+_F, _I, _Z = C.c_float, C.c_int, C.c_size_t
+# the 24-symbol ABI of native-c:src/jvector_simd_kernel_list.h: name -> (restype, argtypes)
+REF_SIGNATURES = {
+    "cosine_f32": (_F, [f32p, _Z, f32p, _Z, _Z]), "dot_product_f32": (_F, [f32p, _Z, f32p, _Z, _Z]),
+    "euclidean_f32": (_F, [f32p, _Z, f32p, _Z, _Z]),
+    "assemble_and_sum_f32": (_F, [f32p, _I, u8p, _I, _Z]), "assemble_and_sum_pq_f32": (_F, [f32p, _Z, u8p, _I, u8p, _I, _I]),
+    "pq_decoded_cosine_similarity_f32": (_F, [u8p, _I, _Z, _I, f32p, f32p, _F]),
+    "calculate_partial_sums_dot_f32": (None, [f32p, _I, _Z, _I, f32p, _I, f32p]),
+    "calculate_partial_sums_euclidean_f32": (None, [f32p, _I, _Z, _I, f32p, _I, f32p]),
+    "calculate_partial_sums_self_magnitude_f32": (None, [f32p, _I, _Z, _I, f32p]),
+    "nvq_quantize_8bit": (None, [f32p, _Z, _F, _F, _F, _F, u8p]), "nvq_loss": (_F, [f32p, _Z, _F, _F, _F, _F, _I]),
+    "nvq_uniform_loss": (_F, [f32p, _Z, _F, _F, _I]),
+    "nvq_square_l2_distance_8bit": (_F, [f32p, u8p, _Z, _F, _F, _F, _F]), "nvq_dot_product_8bit": (_F, [f32p, u8p, _Z, _F, _F, _F, _F]),
+    "nvq_cosine_8bit_packed": (C.c_int64, [f32p, u8p, _Z, _F, _F, _F, _F, f32p]),
+    "nvq_shuffle_query_in_place_8bit": (None, [f32p, _Z]),
+    "add_in_place_f32": (None, [f32p, f32p, _Z]), "sub_in_place_f32": (None, [f32p, f32p, _Z]), "min_in_place_f32": (None, [f32p, f32p, _Z]),
+    "add_scalar_in_place_f32": (None, [f32p, _F, _Z]), "sub_scalar_in_place_f32": (None, [f32p, _F, _Z]),
+    "max_f32": (_F, [f32p, _Z]),
+    "jvector_simd_get_active_isa": (C.c_char_p, []), "jvector_simd_get_max_isa_env": (C.c_char_p, []),
+}
+
+
 def load_ref():
-    """The reference's own libjvector.so, with the 24-symbol ABI of native-c:src/jvector_simd_kernel_list.h."""
+    """The reference's own libjvector.so (built by build() where the reference's sources are present), or None."""
     if not os.path.exists(REF_SO):
-        if os.path.isdir("/root/reference/jvector-native"):
-            build()
-        else:
+        build()
+        if not os.path.exists(REF_SO):
             return None
     L = C.CDLL(REF_SO)
-    F, I, Z = C.c_float, C.c_int, C.c_size_t
-    for n in ("cosine_f32", "dot_product_f32", "euclidean_f32"):
-        getattr(L, n).restype = F
-        getattr(L, n).argtypes = [f32p, Z, f32p, Z, Z]
-    L.assemble_and_sum_f32.restype = F
-    L.assemble_and_sum_f32.argtypes = [f32p, I, u8p, I, Z]
-    L.assemble_and_sum_pq_f32.restype = F
-    L.assemble_and_sum_pq_f32.argtypes = [f32p, Z, u8p, I, u8p, I, I]
-    L.pq_decoded_cosine_similarity_f32.restype = F
-    L.pq_decoded_cosine_similarity_f32.argtypes = [u8p, I, Z, I, f32p, f32p, F]
-    for n in ("calculate_partial_sums_dot_f32", "calculate_partial_sums_euclidean_f32"):
-        getattr(L, n).restype = None
-        getattr(L, n).argtypes = [f32p, I, Z, I, f32p, I, f32p]
-    L.calculate_partial_sums_self_magnitude_f32.restype = None
-    L.calculate_partial_sums_self_magnitude_f32.argtypes = [f32p, I, Z, I, f32p]
-    L.nvq_quantize_8bit.restype = None
-    L.nvq_quantize_8bit.argtypes = [f32p, Z, F, F, F, F, u8p]
-    L.nvq_loss.restype = F
-    L.nvq_loss.argtypes = [f32p, Z, F, F, F, F, I]
-    L.nvq_uniform_loss.restype = F
-    L.nvq_uniform_loss.argtypes = [f32p, Z, F, F, I]
-    for n in ("nvq_square_l2_distance_8bit", "nvq_dot_product_8bit"):
-        getattr(L, n).restype = F
-        getattr(L, n).argtypes = [f32p, u8p, Z, F, F, F, F]
-    L.nvq_cosine_8bit_packed.restype = C.c_int64
-    L.nvq_cosine_8bit_packed.argtypes = [f32p, u8p, Z, F, F, F, F, f32p]
-    L.nvq_shuffle_query_in_place_8bit.restype = None
-    L.nvq_shuffle_query_in_place_8bit.argtypes = [f32p, Z]
-    for n in ("add_in_place_f32", "sub_in_place_f32", "min_in_place_f32"):
-        getattr(L, n).restype = None
-        getattr(L, n).argtypes = [f32p, f32p, Z]
-    for n in ("add_scalar_in_place_f32", "sub_scalar_in_place_f32"):
-        getattr(L, n).restype = None
-        getattr(L, n).argtypes = [f32p, F, Z]
-    L.max_f32.restype = F
-    L.max_f32.argtypes = [f32p, Z]
-    L.jvector_simd_get_active_isa.restype = C.c_char_p
-    L.jvector_simd_get_max_isa_env.restype = C.c_char_p
+    for name, (res, args) in REF_SIGNATURES.items():
+        fn = getattr(L, name)
+        fn.restype = res
+        fn.argtypes = args
     return L
 
 

@@ -32,6 +32,24 @@ def test_recall_at_k_matches_accuracy_metrics_semantics():
     assert bench.recall_at_k(found, truth, 2) == (1 + 0) / 4.0
 
 
+def test_dump_outputs_dtypes_and_seeded_row_sample(tmp_path, monkeypatch):
+    import bench
+    nodes = np.arange(1000 * 10, dtype=np.int32).reshape(1000, 10)
+    scores = np.linspace(0, 1, 10000, dtype=np.float32).reshape(1000, 10)
+    bench.dump_outputs(str(tmp_path / "all"), {"c2_nodes": nodes, "c2_scores": scores})
+    assert np.load(tmp_path / "all" / "c2_nodes.npy").dtype == np.float64
+    assert np.array_equal(np.load(tmp_path / "all" / "c2_nodes.npy"), nodes) and np.array_equal(np.load(tmp_path / "all" / "c2_scores.npy"), scores)
+    # over the cap: the same seeded rows of every array, within the cap, and the same rows run after run
+    monkeypatch.setattr(bench, "DUMP_BYTES", 8192)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"c2_nodes": nodes, "c2_scores": scores})
+    n, s = np.load(tmp_path / "a" / "c2_nodes.npy"), np.load(tmp_path / "a" / "c2_scores.npy")
+    assert n.dtype == np.float64 and s.dtype == np.float32 and 0 < len(n) == len(s) and n.nbytes + s.nbytes <= 8192
+    rows = (n[:, 0] // 10).astype(np.int64)
+    assert np.array_equal(nodes[rows], n) and np.array_equal(scores[rows], s)
+    assert np.array_equal(np.load(tmp_path / "b" / "c2_nodes.npy"), n)
+
+
 def test_measured_peaks_and_traffic_table():
     import bench
     peak, src = bench.measured_peaks()

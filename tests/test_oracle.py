@@ -10,6 +10,7 @@ import pytest
 
 import oracle_lib as o
 from oracle_lib import bp, fp, ip, lp, wp
+from recorded_ref import where_recorded
 
 REL = 1e-4  # native-c:tests/test_similarity.cpp:101,140,172
 
@@ -107,7 +108,8 @@ def test_pq_vs_ref(oracle, ref, dim, M):
         for m in range(M):
             cbm = np.ascontiguousarray(cb[k * offsets[m]: k * (offsets[m] + sizes[m])])
             fn(fp(cbm), m, int(sizes[m]), k, fp(q), int(offsets[m]), fp(rl))
-        np.testing.assert_allclose(lut, rl, rtol=1e-5, atol=1e-6)
+        w = where_recorded(rl)
+        np.testing.assert_allclose(lut[w], rl[w], rtol=1e-5, atol=1e-6)
         for i in range(0, 300, 13):
             want = ref.assemble_and_sum_f32(fp(rl), k, bp(codes), i * M, M)
             got = oracle.jvo_pq_adc(fp(lut), k, bp(codes[i]), M)
@@ -119,7 +121,8 @@ def test_pq_vs_ref(oracle, ref, dim, M):
     for m in range(M):
         cbm = np.ascontiguousarray(cb[k * offsets[m]: k * (offsets[m] + sizes[m])])
         ref.calculate_partial_sums_self_magnitude_f32(fp(cbm), m, int(sizes[m]), k, fp(rmag))
-    np.testing.assert_allclose(mag, rmag, rtol=1e-5, atol=1e-7)
+    w = where_recorded(rmag)
+    np.testing.assert_allclose(mag[w], rmag[w], rtol=1e-5, atol=1e-7)
     lut = np.empty(M * k, np.float32)
     oracle.jvo_pq_lut(fp(cb), ip(sizes), ip(offsets), M, k, None, fp(q), dim, o.DOT_PRODUCT, fp(lut))
     bmag = oracle.jvo_dot_f32(fp(q), fp(q), dim)
@@ -309,22 +312,28 @@ def test_scorer_contexts_port_equals_ref(oracle, ref):
     for i in range(n):
         oracle.jvo_nvq_encode(fp(data[i]), fp(mean), dim, nsub, 1, fp(params[i]), bp(bys[i]))
     q = o.random_unit_vectors(rng, 1, dim)[0]
-    res = {}
-    for use_ref in (False, True):
-        assert oracle.jvo_use_ref(o.REF_SO.encode() if use_ref else None) == 0
-        for metric in (o.EUCLIDEAN, o.DOT_PRODUCT, o.COSINE):
-            ctxs = {"f32": oracle.jvo_scorer_f32(metric, fp(data), n, dim, fp(q)),
-                    "pq": oracle.jvo_scorer_pq(metric, fp(cb), M, k, dim, None, bp(codes), n, fp(q)),
-                    "nvq": oracle.jvo_scorer_nvq(metric, fp(mean), dim, nsub, fp(params), bp(bys), n, fp(q))}
-            for name, c in ctxs.items():
-                res[(use_ref, metric, name)] = np.array([oracle.jvo_scorer_score(c, i) for i in range(n)], np.float32)
+    metrics, kinds = (o.EUCLIDEAN, o.DOT_PRODUCT, o.COSINE), ("f32", "pq", "nvq")
+
+    def scores(ref_so):
+        """[metric][kind][node] scores of the oracle's scorers, their arithmetic routed through ref_so (None: the oracle's own)"""
+        assert oracle.jvo_use_ref(ref_so) == 0
+        out = np.empty((len(metrics), len(kinds), n), np.float32)
+        for a, metric in enumerate(metrics):
+            ctxs = [oracle.jvo_scorer_f32(metric, fp(data), n, dim, fp(q)),
+                    oracle.jvo_scorer_pq(metric, fp(cb), M, k, dim, None, bp(codes), n, fp(q)),
+                    oracle.jvo_scorer_nvq(metric, fp(mean), dim, nsub, fp(params), bp(bys), n, fp(q))]
+            for b, c in enumerate(ctxs):
+                out[a, b] = [oracle.jvo_scorer_score(c, i) for i in range(n)]
                 oracle.jvo_scorer_free(c)
-    oracle.jvo_use_ref(None)
-    for metric in (o.EUCLIDEAN, o.DOT_PRODUCT, o.COSINE):
-        for name in ("f32", "pq", "nvq"):
-            np.testing.assert_allclose(res[(False, metric, name)], res[(True, metric, name)], rtol=1e-5, atol=1e-6)
+        oracle.jvo_use_ref(None)
+        return out
+    port = scores(None)
+    via_ref = ref.capture(lambda: scores(o.REF_SO.encode()))
+    for a in range(len(metrics)):
+        for b in range(len(kinds)):
+            np.testing.assert_allclose(port[a, b], via_ref[a, b], rtol=1e-5, atol=1e-6)
     # the f32 scorer equals jvo_compare
-    assert res[(False, o.DOT_PRODUCT, "f32")][3] == oracle.jvo_compare_f32(o.DOT_PRODUCT, fp(q), fp(data[3]), dim)
+    assert port[metrics.index(o.DOT_PRODUCT), kinds.index("f32")][3] == oracle.jvo_compare_f32(o.DOT_PRODUCT, fp(q), fp(data[3]), dim)
 
 
 def test_retain_diverse_known_answer(oracle):
