@@ -119,6 +119,15 @@ JV_API int jv_dataset_register_nvq(const uint8_t *bytes, const float *params, in
 /* rows already in HBM on the calling thread's device (e.g. produced by another kernel): BORROWED, not copied — the caller keeps
  * them alive until jv_dataset_free. 16-byte aligned, row_stride = dim rounded up to 4 floats, padding floats zero. */
 JV_API int jv_dataset_adopt_f32_device(const float *rows_device, int64_t n, int dim, int row_stride, jv_dataset *out);
+/* fp32 data sets searched with DOT_PRODUCT (dim >= 256, rows >= 252 MB) carry a projection sketch: 32 fp32 projections and two
+ * norms per row (136 bytes per row, in HBM), built by the first such graph search, with which the walk proves most candidates
+ * cannot enter its list without reading their rows. Results are the same with and without it. The sketch describes the rows as
+ * they were when it was built: rows must not change while a data set is in use (adopted rows are the caller's memory) unless
+ * jv_dataset_invalidate_sketch is called after the change and before the next search. JV_F32_SKETCH=0 turns the sketch off. */
+JV_API int jv_dataset_invalidate_sketch(jv_dataset ds);
+/* state: 1 built, 0 not built (yet), -1 skipped because the basis captured < 50 % of the rows' energy (nothing would be dropped);
+ * captured: that share. Any output may be NULL; basis_out [32][row_stride], proj_out [n][32], norms_out [n][2] need state 1. */
+JV_API int jv_dataset_f32_sketch(jv_dataset ds, int *state, double *captured, float *basis_out, float *proj_out, float *norms_out);
 JV_API int jv_dataset_device(jv_dataset ds);
 /* ImmutablePQVectors' code-vs-code scoring (base:quantization/ImmutablePQVectors.java:63-105): build the triangular
  * centroid-vs-centroid table of ProductQuantization.createCodebookPartialSums (ProductQuantization.java:609-628; 12.6 MB at M = 96,
@@ -327,6 +336,7 @@ JV_API int jv_host_register(void *p, size_t bytes); /* pin a host buffer for fas
 JV_API int jv_host_unregister(void *p);
 JV_API int jv_device_synchronize(void);
 JV_API int64_t jv_kernel_launch_count(void); /* kernels this library has launched since load */
+JV_API int64_t jv_search_rows_read(void);    /* fp32 rows the graph searches' walks have read since load (< visited with a sketch) */
 
 #ifdef __cplusplus
 }

@@ -44,6 +44,8 @@ public:
     int64_t size() const { return jv_dataset_size(h_); }
     int dimension() const { return jv_dataset_dim(h_); }
     jv_dataset handle() const { return h_; }
+    // fp32 rows changed in place (adopted device rows): the projection sketch no longer describes them (jv_dataset_invalidate_sketch)
+    void invalidate_sketch() { jv_dataset_invalidate_sketch(h_); }
     /// BuildScoreProvider.diversityProviderFor: score(a[i], b[i]) for every pair, one launch
     std::vector<float> diversityScores(const std::vector<int32_t> &a, const std::vector<int32_t> &b, VectorSimilarityFunction vsf) const
     {

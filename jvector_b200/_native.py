@@ -63,6 +63,7 @@ SYMBOLS = [
     ("jv_dataset_register_bq", _I, [u64p, _L, _I, C.POINTER(_P)]),
     ("jv_dataset_register_nvq", _I, [u8p, f32p, _L, _I, _I, f32p, C.POINTER(_P)]),
     ("jv_dataset_adopt_f32_device", _I, [_P, _L, _I, _I, C.POINTER(_P)]), ("jv_dataset_device", _I, [_P]),
+    ("jv_dataset_invalidate_sketch", _I, [_P]), ("jv_dataset_f32_sketch", _I, [_P, C.POINTER(_I), C.POINTER(C.c_double), f32p, f32p, f32p]),
     ("jv_dataset_pq_pair_table", _I, [_P, _I]), ("jv_dataset_pq_pair_table_download", _I, [_P, _I, f32p]),
     ("jv_dataset_free", _I, [_P]), ("jv_dataset_size", _L, [_P]), ("jv_dataset_dim", _I, [_P]), ("jv_dataset_device_bytes", _L, [_P]),
     ("jv_query_begin", _I, [_P, f32p, _I, C.POINTER(_P)]), ("jv_score_batch", _I, [_P, i32p, _I, f32p]), ("jv_query_end", _I, [_P]),
@@ -101,7 +102,7 @@ SYMBOLS = [
     ("jv_builder_finish", _I, [_P, C.POINTER(_P), C.POINTER(C.c_double)]), ("jv_builder_free", _I, [_P]),
     ("jv_device_malloc", _I, [C.POINTER(_P), _Z]), ("jv_device_free", _I, [_P]), ("jv_memcpy_h2d", _I, [_P, _P, _Z]),
     ("jv_memcpy_d2h", _I, [_P, _P, _Z]), ("jv_host_register", _I, [_P, _Z]), ("jv_host_unregister", _I, [_P]),
-    ("jv_device_synchronize", _I, []), ("jv_kernel_launch_count", _L, []),
+    ("jv_device_synchronize", _I, []), ("jv_kernel_launch_count", _L, []), ("jv_search_rows_read", _L, []),
 ]
 
 _lib = None

@@ -10,7 +10,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.environ.get("JV_B200_LIBDIR") or os.path.join(HERE, "lib")
 SO = os.path.join(LIBDIR, "libjvector_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-CU = ["kernels_batch.cu", "bq_imma.cu", "bq_umma.cu", "search.cu", "build.cu", "api.cu"]
+CU = ["kernels_batch.cu", "bq_imma.cu", "bq_umma.cu", "search.cu", "sketch.cu", "build.cu", "api.cu"]
 CPP = ["legacy_host.cpp", "legacy_simd.cpp", "legacy_avx512.cpp"]
 HEADERS = ["common.cuh", "scorers.cuh", "kernels.h", "legacy_avx512.h", os.path.join("..", "..", "include", "jvector_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

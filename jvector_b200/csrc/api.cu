@@ -158,6 +158,13 @@ struct jv_dataset_s {
     DataDesc d;
     std::vector<void *> allocs;
     size_t bytes = 0;
+    // fp32 DOT_PRODUCT walks: the projection sketch (kernels.h F32Sketch), built by the first search that can use it. Handles are
+    // shared across threads: sketch_mu guards the build and jv_dataset_invalidate_sketch.
+    std::mutex sketch_mu;
+    int sketch_state = 0;  // 0 not built, 1 built, -1 skipped: the basis captured too little of the rows' energy to drop anything
+    double sketch_captured = 0.0;
+    void *sketch_mem = nullptr;
+    F32Sketch sketch = {};
     int alloc(void **p, size_t n)
     {
         CK(cudaMalloc(p, n ? n : 16), "cudaMalloc(dataset)");
@@ -168,6 +175,7 @@ struct jv_dataset_s {
     ~jv_dataset_s()
     {
         for (void *p : allocs) cudaFree(p);
+        if (sketch_mem) cudaFree(sketch_mem);
     }
 };
 
@@ -313,6 +321,8 @@ const char *jv_last_error(void) { return t_err.c_str(); }
 const char *jv_version(void) { return "jvector-b200 0.1 (sm_100a)"; }
 int jv_gpu_sm_count(void) { return g_default_device >= 0 ? g_sm_counts[t_device >= 0 ? t_device : g_default_device] : 0; }
 int64_t jv_kernel_launch_count(void) { return (int64_t)g_launches.load(); }
+static std::atomic<long long> g_rows_read{0};
+int64_t jv_search_rows_read(void) { return (int64_t)g_rows_read.load(); }
 
 // ------------------------------------------------------------------------------------------------ data sets
 int jv_dataset_register_f32(const float *rows, int64_t n, int dim, jv_dataset *out)
@@ -514,6 +524,32 @@ int jv_dataset_free(jv_dataset ds)
     delete ds;
     return JV_OK;
 }
+int jv_dataset_invalidate_sketch(jv_dataset ds)
+{
+    ON_DEVICE_OF(ds);
+    std::lock_guard<std::mutex> lk(ds->sketch_mu);
+    CK(cudaDeviceSynchronize(), "invalidate_sketch: synchronize");
+    if (ds->sketch_mem) cudaFree(ds->sketch_mem);
+    ds->sketch_mem = nullptr;
+    ds->sketch = {};
+    ds->sketch_state = 0;
+    return JV_OK;
+}
+
+int jv_dataset_f32_sketch(jv_dataset ds, int *state, double *captured, float *basis_out, float *proj_out, float *norms_out)
+{
+    ON_DEVICE_OF(ds);
+    std::lock_guard<std::mutex> lk(ds->sketch_mu);
+    if (state) *state = ds->sketch_state;
+    if (captured) *captured = ds->sketch_captured;
+    if (!basis_out && !proj_out && !norms_out) return JV_OK;
+    if (ds->sketch_state != 1) return fail(JV_ERR_INVALID, "f32_sketch: the data set has no sketch");
+    if (basis_out) CK(cudaMemcpy(basis_out, ds->sketch.basis, (size_t)SKETCH_K * ds->d.stride * 4, cudaMemcpyDeviceToHost), "D2H sketch basis");
+    if (proj_out) CK(cudaMemcpy(proj_out, ds->sketch.proj, (size_t)ds->d.n * SKETCH_K * 4, cudaMemcpyDeviceToHost), "D2H sketch projections");
+    if (norms_out) CK(cudaMemcpy(norms_out, ds->sketch.norms, (size_t)ds->d.n * 8, cudaMemcpyDeviceToHost), "D2H sketch norms");
+    return JV_OK;
+}
+
 int64_t jv_dataset_size(jv_dataset ds) { return ds ? ds->d.n : 0; }
 int jv_dataset_dim(jv_dataset ds) { return ds ? ds->d.dim : 0; }
 int64_t jv_dataset_device_bytes(jv_dataset ds) { return ds ? (int64_t)ds->bytes : 0; }
@@ -1068,6 +1104,38 @@ int jv_graph_download(jv_graph g, int level, int32_t *node_ids_out, int32_t *adj
     return JV_OK;
 }
 
+// The sketch pays where a walk's rows come from HBM: rows of at least 1 KB (a sketch line + norms cost 160 bytes of reads) and a data
+// set of at least twice the 126 MB L2. JV_F32_SKETCH=0 turns it off.
+static bool sketch_wanted(const jv_dataset approx, int metric)
+{
+    if (approx->d.kind != KIND_F32 || metric != JV_METRIC_DOT || approx->d.dim < 256) return false;
+    if ((double)approx->d.n * approx->d.stride * 4 < 2.0 * 126e6) return false;
+    const char *e = getenv("JV_F32_SKETCH");
+    return !(e && e[0] == '0');
+}
+
+static int sketch_ensure(jv_dataset ds, cudaStream_t s)
+{
+    std::lock_guard<std::mutex> lk(ds->sketch_mu);
+    if (ds->sketch_state != 0) return JV_OK;
+    const size_t bytes = f32_sketch_bytes(ds->d);
+    CK(cudaMalloc(&ds->sketch_mem, bytes), "cudaMalloc(sketch)");
+    cudaError_t e = build_f32_sketch(ds->d, ds->sketch_mem, &ds->sketch, &ds->sketch_captured, s);
+    if (e != cudaSuccess) {
+        cudaFree(ds->sketch_mem);
+        ds->sketch_mem = nullptr;
+        return cuda_fail(e, "build_f32_sketch");
+    }
+    // 32 of 768 directions of i.i.d. rows hold ~4 % of their energy: the bound would drop nothing and cost 160 bytes a candidate
+    if (ds->sketch_captured < 0.5) {
+        cudaFree(ds->sketch_mem);
+        ds->sketch_mem = nullptr;
+        ds->sketch = {};
+        ds->sketch_state = -1;
+    } else ds->sketch_state = 1;
+    return JV_OK;
+}
+
 static int search_device(jv_graph g, jv_dataset approx, jv_dataset reranker, int metric, const float *queries_dev, int nq, int topK, int rerankK,
                          const SearchFilter *filter, int32_t *nodes_dev, float *scores_dev, jv_search_stats *stats)
 {
@@ -1084,6 +1152,11 @@ static int search_device(jv_graph g, jv_dataset approx, jv_dataset reranker, int
     if ((rc = t_ctx.init())) return rc;
     cudaStream_t s = t_ctx.stream;
     const DataDesc *rr = reranker ? &reranker->d : nullptr;
+    const F32Sketch *sketch = nullptr;
+    if (sketch_wanted(approx, metric)) {
+        if ((rc = sketch_ensure(approx, s))) return rc;
+        if (approx->sketch_state == 1) sketch = &approx->sketch;
+    }
     SearchPlan plan;
     // JV_VISITED_CAP / JV_LIST_CAP: first visited-table / candidate-list sizes (testing and tuning knobs; queries that outgrow
     // either are re-run below with 4x)
@@ -1100,7 +1173,8 @@ static int search_device(jv_graph g, jv_dataset approx, jv_dataset reranker, int
     int32_t *dindex = (int32_t *)(a + sizeof(SearchCounters) + 64 + (((size_t)nq + 63) & ~(size_t)63));
     CK(cudaMemsetAsync(dcnt, 0, sizeof(SearchCounters), s), "memset counters");
     CK(cudaEventRecord(t_ctx.ev0, s), "event");
-    CK(launch_search(g->g, approx->d, rr, metric, queries_dev, nq, topK, rerankK, plan, t_ctx.dbuf[5], dwork, nodes_dev, scores_dev, dcnt, dover, nullptr, 0, filter, s),
+    CK(launch_search(g->g, approx->d, rr, metric, queries_dev, nq, topK, rerankK, plan, t_ctx.dbuf[5], dwork, nodes_dev, scores_dev, dcnt, dover, nullptr, 0, filter, s,
+                     sketch),
        "launch_search");
     CK(cudaEventRecord(t_ctx.ev1, s), "event");
     SearchCounters hc;
@@ -1138,7 +1212,7 @@ static int search_device(jv_graph g, jv_dataset approx, jv_dataset reranker, int
         CK(cudaMemcpyAsync(&dcnt->overflowed, &zero, sizeof(zero), cudaMemcpyHostToDevice, s), "reset overflow");
         CK(cudaEventRecord(t_ctx.ev0, s), "event");
         CK(launch_search(g->g, approx->d, rr, metric, queries_dev, (int)idx.size(), topK, rerankK, p2, t_ctx.dbuf[5], dwork, nodes_dev, scores_dev, dcnt, dover,
-                         dindex, 0, filter, s),
+                         dindex, 0, filter, s, sketch),
            "launch_search(retry)");
         CK(cudaEventRecord(t_ctx.ev1, s), "event");
         CK(cudaMemcpyAsync(&hc, dcnt, sizeof(hc), cudaMemcpyDeviceToHost, s), "D2H counters");
@@ -1148,6 +1222,7 @@ static int search_device(jv_graph g, jv_dataset approx, jv_dataset reranker, int
         ms += ms2;
     }
     if (hc.overflowed > 0) return fail(JV_ERR_OVERFLOW, "graph_search: visited table / candidate list overflow after retries");
+    g_rows_read += (long long)hc.rows_read;  // the counters add up over the re-runs (only `overflowed` is reset)
     if (stats) {
         stats->visited = (int64_t)hc.visited;
         stats->expanded = (int64_t)hc.expanded;

@@ -64,6 +64,14 @@ __device__ __forceinline__ int group_sum_int(int v)
     return v;
 }
 
+// warp-wide double sum, result in every lane
+__device__ __forceinline__ double warp_sum_d(double v)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
+    return v;
+}
+
 // 128-bit streaming load that bypasses L1 allocation (rows are touched once per query)
 __device__ __forceinline__ float4 ldg_stream(const float4 *p)
 {

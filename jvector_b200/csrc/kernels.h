@@ -31,7 +31,23 @@ struct GraphDesc {
 
 struct SearchCounters {  // device-side totals
     unsigned long long visited, expanded, expanded_base, reranked, overflowed;
+    unsigned long long rows_read;  // fp32 walks: full rows the walking scorer read (visited minus the sketch's drops)
 };
+
+// ---- sketch.cu: projection sketch of an fp32 data set (DOT_PRODUCT walks skip rows it proves cannot enter the list) ----
+// For an orthonormal basis P (SKETCH_K rows of `stride` floats) and r = x - P^T (P x):  q.x = (P q).(P x) + q.r  and
+// q.r <= ||q - P^T P q|| ||r||, so (P q).(P x) + ||q_perp|| ||r|| bounds the score from above for 128 + 8 bytes of reads per row.
+constexpr int SKETCH_K = 32;
+struct F32Sketch {
+    const float *basis;   // [SKETCH_K][stride] fp32 rows of P (orthonormal in double, then rounded)
+    const double *gram;   // [SKETCH_K][SKETCH_K] basis . basis^T of the ROUNDED rows (what the query side's ||q_perp|| uses)
+    const float4 *proj;   // [n][SKETCH_K / 4] fp32(P x): one 128-byte line per row
+    const float2 *norms;  // [n] {||x - P^T fp32(P x)||, ||x||}, both rounded up
+};
+size_t f32_sketch_bytes(const DataDesc &d);
+// builds the sketch of `d` into `mem` (f32_sketch_bytes long) and synchronises `s`. *captured = the share of the sample rows'
+// energy (sum of squares) the basis captures; the caller discards a sketch that captures too little to drop anything.
+cudaError_t build_f32_sketch(const DataDesc &d, void *mem, F32Sketch *sk, double *captured, cudaStream_t s);
 
 // ---- kernels_batch.cu ----
 cudaError_t launch_prepare(const DataDesc &d, int metric, const float *queries_dev, int nq, float *blobs_dev, cudaStream_t s);
@@ -125,7 +141,8 @@ size_t search_scratch_bytes(const SearchPlan &p);
 cudaError_t launch_search(const GraphDesc &g, const DataDesc &approx, const DataDesc *rerank, int metric, const float *queries_dev,
                           int nq, int topK, int rerankK, const SearchPlan &plan, void *scratch_dev, int *work_counter_dev,
                           int32_t *nodes_out_dev, float *scores_out_dev, SearchCounters *counters_dev, uint8_t *overflow_flags_dev,
-                          const int32_t *query_index_dev, int query_stride, const SearchFilter *filter, cudaStream_t s);
+                          const int32_t *query_index_dev, int query_stride, const SearchFilter *filter, cudaStream_t s,
+                          const F32Sketch *sketch = nullptr);
 
 // ---- build.cu ----
 struct BuildParams {

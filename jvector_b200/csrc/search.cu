@@ -64,8 +64,54 @@ struct SearchParams {
     int early_pf;      // request the adjacency / FusedPQ record of a new candidate that lands among the next two pops at score time
     int pq_rows;       // PQ walk: lane = candidate, warp = partial sum (score_pq_partial) instead of an 8-lane group per candidate
     int row_prefetch;  // fp32 / NVQ walks: 1 = a bulk L2 prefetch of every newly visited row is issued by the thread that discovered it
+    int sketch;        // fp32 DOT_PRODUCT walks: `sk` bounds a candidate's score before its row is read (see SKETCH_MARGIN)
+    F32Sketch sk;
     unsigned long long *dbg;  // JV_SEARCH_PROFILE builds only: per-phase cycle totals
 };
+
+// Slack of the sketch bound, relative to ||q|| ||x||. A candidate is dropped unread when
+//     score_map(fp32(P q) . fp32(P x) + ||q_perp|| ||r|| + SKETCH_MARGIN ||q|| ||x||) < score of the list's last entry,
+// which is sound when the margin covers every gap between that sum and the fp32 score the row scorer would have produced:
+//   * the row scorer's 768-term fp32 dot: at most gamma_768 = 768 * 2^-24 = 4.6e-5 of ||q|| ||x|| (sum |q_i x_i| <= ||q|| ||x||);
+//   * the 32-term fp32 dot of the sketch, with P q and P x each rounded once from double: ~(32 + 2) * 2^-24 = 2e-6;
+//   * P rounded to fp32 is orthonormal only to ~32 * 2^-23 = 3.8e-6, which P^T r != 0 costs at most ~4e-6 (||q_perp|| itself is
+//     exact: it is measured against the Gram matrix of the rounded basis);
+//   * ||q_perp||, ||q||, ||r||, ||x|| are rounded UP from double, and the three fp32 additions of the bound cost a few 2^-24.
+// Total below 6e-5; 1e-3 keeps a factor of 15 in hand and drops ~0.1 % fewer candidates than the exact test would.
+constexpr float SKETCH_MARGIN = 1e-3f;
+
+// whole CTA: out[0..SKETCH_K) = fp32(P q), out[SKETCH_K] = ||q - P^T P q||, out[SKETCH_K + 1] = ||q||, from the prepared fp32 query
+// in shared memory. In double: with a = P q, ||q - P^T a||^2 = ||q||^2 - 2 a.a + a^T G a, G the Gram matrix of the stored basis.
+__device__ __forceinline__ void sketch_prepare(const F32Sketch &sk, int stride, const float *q, float *out, double *dred)
+{
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+    for (int j = warp; j < SKETCH_K; j += nw) {
+        const float *b = sk.basis + (size_t)j * stride;
+        double a = 0.0;
+        for (int i = lane; i < stride; i += 32) a = fma((double)__ldg(b + i), (double)q[i], a);
+        a = warp_sum_d(a);
+        if (lane == 0) dred[j] = a;
+    }
+    double qq = 0.0;
+    for (int i = tid; i < stride; i += blockDim.x) qq = fma((double)q[i], (double)q[i], qq);
+    qq = warp_sum_d(qq);
+    if (lane == 0) dred[SKETCH_K + warp] = qq;
+    __syncthreads();
+    if (warp == 0) {
+        const double a = dred[lane];
+        double t = 0.0;
+        for (int k = 0; k < SKETCH_K; k++) t = fma(__ldg(sk.gram + lane * SKETCH_K + k), dred[k], t);
+        const double aa = warp_sum_d(a * a), aga = warp_sum_d(a * t);
+        double q2 = 0.0;
+        for (int w = 0; w < nw; w++) q2 += dred[SKETCH_K + w];
+        out[lane] = (float)a;
+        if (lane == 0) {
+            out[SKETCH_K] = __double2float_ru(sqrt(fmax(0.0, q2 - 2.0 * aa + aga)));
+            out[SKETCH_K + 1] = __double2float_ru(sqrt(q2));
+        }
+    }
+    __syncthreads();
+}
 
 __device__ __forceinline__ bool visited_insert(int32_t *t, unsigned mask, int shift, int32_t v)
 {
@@ -250,6 +296,11 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
     __shared__ int s_q, s_n, s_m, s_hsize, s_cnt;
     __shared__ int s_drop[2];  // best sortable score that fell off the list, double-buffered like s_posv
     __shared__ int s_posv[2];
+    // fp32 sketch: P q, ||q_perp||, ||q|| (sketch_prepare) and the count of a hop's candidates the bound did not drop. The survivors'
+    // ids go to the idle list buffer `nxt` (written only by the merge; launch_search checks that it holds a whole hop), and
+    // sketch_prepare's scratch to cand_keys (idle before the walk): 9 CTAs per SM leave no room for more static shared memory.
+    __shared__ __align__(16) float s_sk[KIND == KIND_F32 ? SKETCH_K + 4 : 4];
+    __shared__ int s_ns;
 
     const int tid = threadIdx.x;
     const int group = tid / G, lane = tid % G;
@@ -285,6 +336,7 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
 #endif
         JV_T(t_q0);
         prepare_blob(P.approx, P.metric, q, blobA, red, blobH, splitm);
+        if (KIND == KIND_F32 && P.sketch) sketch_prepare(P.sk, P.approx.stride, blobA, s_sk, reinterpret_cast<double *>(cand_keys));
         if (P.has_rerank) prepare_blob(P.rerank, P.metric, q, blobR, red);
         if (vsm) {
             int4 *t4 = reinterpret_cast<int4 *>(vis);
@@ -315,7 +367,7 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
         }
         int size = 1;
         int table_cnt = 1;
-        unsigned visited = 0, expanded = 0, expanded_base = 0;
+        unsigned visited = 0, expanded = 0, expanded_base = 0, rows_read = 0;
         int failed = 0;  // 1: visited table full, 2: candidate list too short for a tie tail
         bool truncated = false, inexact = false;  // lenient mode: the walk was cut short / a tie tail was dropped
         __syncthreads();
@@ -325,7 +377,7 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
             // a new level: results + evicted are candidates again (setEntryPointsFromPreviousLayer), the result heap is empty
             for (int i = tid; i < size; i += SEARCH_THREADS) fcur[i] &= F_ACCEPTED;
             int sel = 0;
-            if (tid == 0) { s_posv[0] = 0; s_posv[1] = INT_MAX; s_n = 0; s_m = 0; s_hsize = 0; s_drop[0] = INT_MIN; s_drop[1] = INT_MIN; s_cnt = 0; }
+            if (tid == 0) { s_posv[0] = 0; s_posv[1] = INT_MAX; s_n = 0; s_m = 0; s_hsize = 0; s_drop[0] = INT_MIN; s_drop[1] = INT_MIN; s_cnt = 0; s_ns = 0; }
             __syncthreads();
             for (;;) {
                 const int p = s_posv[sel];  // first unexpanded entry = the top of the candidate queue
@@ -341,6 +393,8 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
                 int action = 0;
                 if (lvl > 0 || (fcur[p] & F_ACCEPTED)) action = hs < K ? 1 : (csc > wsc ? 2 : 3);
                 const int dead = (lvl > 0 && action == 3) ? p : -1;
+                // a full list at level 0: a candidate can only enter it by beating the last entry, which the sketch bound tests first
+                const bool skh = KIND == KIND_F32 && P.sketch && lvl == 0 && size == LC;
                 if (tid == 0) { fcur[p] |= F_EXPANDED; s_posv[sel ^ 1] = INT_MAX; s_m = 0; }
                 expanded++;
                 if (lvl == 0) expanded_base++;
@@ -382,7 +436,11 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
                             if (KIND == KIND_PQ) cand_slot[slot] = (uint8_t)t;
                             // the row is needed one barrier from now: start the DRAM -> L2 transfer of all of it at once (one
                             // UBLKPF per row; bytes in flight that occupy no registers and no shared memory)
-                            if (KIND == KIND_F32 && P.row_prefetch == 1) bulk_prefetch_l2(P.approx.rows + (size_t)f * P.approx.stride, (unsigned)P.approx.stride * 4u);
+                            if (KIND == KIND_F32 && skh) {
+                                // the bound needs the 128-byte sketch line and the norms; the row only if the candidate survives
+                                prefetch_l2(P.sk.proj + (size_t)f * (SKETCH_K / 4));
+                                prefetch_l2(P.sk.norms + f);
+                            } else if (KIND == KIND_F32 && P.row_prefetch == 1) bulk_prefetch_l2(P.approx.rows + (size_t)f * P.approx.stride, (unsigned)P.approx.stride * 4u);
                             if (KIND == KIND_NVQ && P.row_prefetch == 1) {
                                 bulk_prefetch_l2(P.approx.bytes + (size_t)f * P.approx.byte_stride, (unsigned)P.approx.byte_stride);
                                 prefetch_l2(P.approx.params + (size_t)f * 4 * P.approx.nsub);  // {min, max, growthRate, midpoint} per sub-vector
@@ -479,11 +537,41 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
         }                                                                                                                           \
     } while (0)
                 if (KIND == KIND_F32) {
+                    const int32_t *ids = cand_ids;
+                    int ns = n;
+                    if (skh) {
+                        // bound pass: 8 lanes per candidate, one 16-byte piece of its sketch line each. A candidate whose bound is under
+                        // the last entry is dropped here exactly as JV_EMIT would drop it after reading the row; the bound, not the
+                        // unread exact score, goes into s_drop (>= the exact score, so the exactness test below stays sound). The rows
+                        // of the survivors are requested at once and scored by the unchanged loop below.
+                        const float tail = key_score(cur[LC - 1]);
+                        const int sl = tid & 7;
+                        int32_t *surv = reinterpret_cast<int32_t *>(nxt);
+                        for (int i = tid >> 3; i < n; i += SEARCH_THREADS / 8) {
+                            const int32_t f = cand_ids[i];
+                            const float4 u = __ldg(P.sk.proj + (size_t)f * (SKETCH_K / 4) + sl);
+                            const float4 a = reinterpret_cast<const float4 *>(s_sk)[sl];
+                            const float d = group_sum<8>(fmaf(a.x, u.x, fmaf(a.y, u.y, fmaf(a.z, u.z, __fmul_rn(a.w, u.w)))));
+                            if (sl == 0) {
+                                const float2 nm = __ldg(P.sk.norms + f);
+                                const float ub = score_map(METRIC, d + s_sk[SKETCH_K] * nm.x + SKETCH_MARGIN * s_sk[SKETCH_K + 1] * nm.y);
+                                if (ub < tail) atomicMax(&s_drop[sel], float_to_sortable(ub));
+                                else {
+                                    surv[atomicAdd(&s_ns, 1)] = f;
+                                    bulk_prefetch_l2(P.approx.rows + (size_t)f * P.approx.stride, (unsigned)P.approx.stride * 4u);
+                                }
+                            }
+                        }
+                        __syncthreads();
+                        ids = surv;
+                        ns = s_ns;
+                    }
+                    rows_read += ns;
                     // two rows per warp at a time: twice the loads in flight, query fragment read once
-                    for (int i = group; i < n; i += 2 * NG) {
-                        const int32_t fa = cand_ids[i];
-                        const bool two = i + NG < n;
-                        const int32_t fb = two ? cand_ids[i + NG] : fa;
+                    for (int i = group; i < ns; i += 2 * NG) {
+                        const int32_t fa = ids[i];
+                        const bool two = i + NG < ns;
+                        const int32_t fb = two ? ids[i + NG] : fa;
                         float sa, sb;
                         score_f32_pair<METRIC>(P.approx, blobA, fa, fb, lane, sa, sb);
                         if (lane == 0) {
@@ -583,7 +671,7 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
                 }
                 if (mypos != INT_MAX) atomicMin(&s_posv[sel ^ 1], mypos);
                 if (mydrop != INT_MIN) atomicMax(&s_drop[sel], mydrop);
-                if (tid == 0) s_n = 0;
+                if (tid == 0) { s_n = 0; s_ns = 0; }
                 __syncthreads();
                 JV_T(t_i3);
                 JV_ACC(3, t_i2, t_i3);
@@ -591,7 +679,8 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
                 if (tid == 0) { dbg_local[5] += 1; dbg_local[6] += (unsigned long long)n; }
 #endif
                 // something fell off the end of the list: that is exact only if at least rerankK accepted entries score strictly
-                // higher than everything dropped (then none of it can be popped before stopSearch fires)
+                // higher than everything dropped (then none of it can be popped before stopSearch fires). For a candidate the sketch
+                // dropped unread, dm holds its bound: the test may fail where the exact score would have passed, never the reverse.
                 const int dm = s_drop[sel];
                 if (dm != INT_MIN) {
                     bool ok;
@@ -742,6 +831,7 @@ __global__ void __launch_bounds__(SearchThreads<KIND>::value, MINB) graph_search
                 atomicAdd(&P.counters->expanded, (unsigned long long)expanded);
                 atomicAdd(&P.counters->expanded_base, (unsigned long long)expanded_base);
                 atomicAdd(&P.counters->reranked, (unsigned long long)reranked);
+                if (KIND == KIND_F32) atomicAdd(&P.counters->rows_read, (unsigned long long)rows_read);
             }
         }
         __syncthreads();
@@ -984,10 +1074,14 @@ size_t search_scratch_bytes(const SearchPlan &p)
 cudaError_t launch_search(const GraphDesc &g, const DataDesc &approx, const DataDesc *rerank, int metric, const float *queries_dev,
                           int nq, int topK, int rerankK, const SearchPlan &plan, void *scratch_dev, int *work_counter_dev,
                           int32_t *nodes_out_dev, float *scores_out_dev, SearchCounters *counters_dev, uint8_t *overflow_flags_dev,
-                          const int32_t *query_index_dev, int query_stride, const SearchFilter *filter, cudaStream_t s)
+                          const int32_t *query_index_dev, int query_stride, const SearchFilter *filter, cudaStream_t s,
+                          const F32Sketch *sketch)
 {
     if (nq <= 0) return cudaSuccess;
     SearchParams P;
+    // (the survivors of a hop, up to `degree` ids, are staged in one idle list buffer of list_alloc 64-bit entries)
+    P.sketch = (sketch && approx.kind == KIND_F32 && metric == JV_METRIC_DOT && 2 * plan.list_alloc >= g.degree) ? 1 : 0;
+    P.sk = P.sketch ? *sketch : F32Sketch{};
     P.accept_bits = filter ? filter->accept_bits : nullptr;
     P.accept_stride = filter ? filter->accept_stride_words : 0;
     P.threshold = filter ? filter->threshold : 0.f;
